@@ -9,12 +9,13 @@ One "step" = one complete sampler call over one batch of synthetic latents per G
     cfg4  sample_euler_ancestral 50 steps + BrownianTreeNoiseSampler, 256x256 neighbourhood model, batch 32 per GPU (256 over 8)
     cfg5  sample_heun 50 steps, 512x512 hourglass depths [2,2,4] widths [256,512,1024], batch 16 per GPU (128 over 8)
 
-    python bench.py [--config cfgN] [--gpus N] [--steps K] [--warmup W]   # N>1: launched by torch.distributed.run
+    python bench.py [--config cfgN] [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # N>1: launched by torch.distributed.run
     python bench.py --impl reference ...                                  # the reference algorithm's CPU port (oracle/)
 
 Weak scaling: every rank samples its own batch.  Prints ONE JSON line on rank 0 (contract: task statement / DESIGN.md section 6).
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -33,6 +34,7 @@ import torch
 
 UNIT = "images/s"
 SIGMA_MIN, SIGMA_MAX = 1e-2, 160.0
+DUMP_LIMIT_BYTES = 64 * 10**6
 _NA_RAW = {"model": {"type": "image_transformer_v2", "input_channels": 3, "input_size": [256, 256], "patch_size": [4, 4],
                      "depths": [2, 2, 4], "widths": [128, 256, 512], "loss_config": "karras", "loss_weighting": "soft-min-snr",
                      "dropout_rate": [0.0, 0.0, 0.1], "augment_prob": 0.0, "sigma_data": 0.5, "sigma_min": 1e-2, "sigma_max": 160,
@@ -71,13 +73,36 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the roofline, parity and cpu_baseline legs")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--parity-seconds", type=float, default=25.0, help="CPU budget of the parity leg (oracle run of one image)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images the last timed step sampled (all ranks, float32) to DIR/samples.npy; beyond "
+                         f"{DUMP_LIMIT_BYTES // 10**6} MB a seeded subset of whole images, their indices in DIR/samples_index.npy")
     args = ap.parse_args()
     args.wl = CONFIGS[args.config]
     if args.batch is None:
         args.batch = args.wl["batch"]
     if args.steps is None:
         args.steps = 3 if args.config == "cfg5" else 5
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference leg times shortened schedules on other inputs)")
     return args
+
+
+def dump_outputs(directory, samples):
+    """samples [N, C, H, W] on the host -> DIR/samples.npy (float32).  The inputs are seeded, so two builds run with the same
+    arguments can be compared file for file; above DUMP_LIMIT_BYTES a fixed seeded subset of whole images is kept."""
+    import numpy as np
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    samples = samples.float()
+    per_image = samples[0].numel() * samples.element_size()
+    if samples.shape[0] * per_image > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // per_image - 1)          # leaves room for the index file
+        idx = torch.randperm(samples.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        samples = samples[idx]
+        np.save(out / "samples_index.npy", idx.double().numpy())
+    np.save(out / "samples.npy", samples.contiguous().numpy())
 
 
 def raw_model_config(wl):
@@ -109,6 +134,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.FIELDS}", "--format=csv,noheader,nounits", "-lms", "200", "-i", str(index)],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)          # the poller must not outlive a bench that fails before stop()
             self.t = threading.Thread(target=self._pump, daemon=True)
             self.t.start()
         except OSError:
@@ -363,17 +389,19 @@ def main():
         t0 = time.time()
         e0.record()
         for i in range(k):
-            fn(i)
+            last = fn(i)
         e1.record()
         barrier()
         t1 = time.time()
-        return max_over_ranks(e0.elapsed_time(e1)), S.total_kernel_launches() - n0, t0, t1
+        return max_over_ranks(e0.elapsed_time(e1)), S.total_kernel_launches() - n0, t0, t1, last
 
     clocks = ClockSampler(local) if rank == 0 else None
     time.sleep(0.3)
-    ms, launches, t0, t1 = timed(step_device, args.steps, args.warmup)
+    ms, launches, t0, t1, last = timed(step_device, args.steps, args.warmup)
     clk = clocks.stop(t0, t1) if clocks else None
-    ms_e2e, _, _, _ = timed(step_e2e, args.steps, 1)
+    dumped = K.parallel.gather_samples(last).cpu() if args.dump_outputs else None
+    del last
+    ms_e2e, _, _, _, _ = timed(step_e2e, args.steps, 1)
     out = step_device(0)
     finite = bool(torch.isfinite(out).all())
     value = world * B * args.steps / (ms / 1000.0)
@@ -523,6 +551,8 @@ def main():
                 "parity_rel_l2": None if not parity else parity.get("rel_l2"),
                 "kernel_breakdown": breakdown, "weights_broadcast_bytes": bcast_bytes, "output_finite": finite,
                 "native_library": str(_native.LIB_PATH.relative_to(ROOT))}
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
